@@ -920,7 +920,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--workload", default="diffuse", choices=["diffuse", "pathtracer"],
                     help="diffuse = configs[2] headline (default); pathtracer = configs[4] 8-bounce path stream")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of the last step's hit records (and the rays they belong to) "
+                         "as DIR/<field>.npy, for comparing two builds output for output (diffuse workload, one GPU)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "diffuse" or args.impl != "b200" or args.gpus != 1
+                              or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs covers the diffuse workload of --impl b200 on one GPU")
     if args.workload == "pathtracer":
         if "--rays" not in sys.argv:
             args.rays = 1 << 25          # paths per GPU; a step traces 16 rays per path
@@ -1064,6 +1070,8 @@ def main():
     value = n * world / (ms_per_step * 1e-3) * 1e-6
     lib.check(dev)
     sampler.join(timeout=2)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, A, B)
     gather_ab = None
     if world > 1 and os.environ.get("RTCB200_GATHER_AB"):   # untimed extra: the same steps with the other delivery mode
         gather_ab = {"default_mode_ms": ms_per_step}
@@ -1259,6 +1267,32 @@ def main():
         emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_RAYS = 1 << 18     # ~21 MB of .npy files
+
+
+def dump_outputs(out_dir, rays_in, rayhits):
+    """Write the RTCRayHit records the timed trace returned ([n, 24] float32 on the device) for a fixed sample of
+    DUMP_RAYS ray indices (seed 0, independent of the run), together with those rays' inputs, as out_dir/<field>.npy.
+    The inputs are written as well because the bounce rays start at the primary hits, i.e. they are computed too."""
+    n = rayhits.shape[0]
+    k = min(n, DUMP_RAYS)
+    idx = np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    sel = torch.from_numpy(idx).to(rayhits.device)
+    hit = rayhits.index_select(0, sel).cpu().numpy()
+    ray = rays_in.index_select(0, sel).cpu().numpy()
+    ids = hit.view(np.uint32)
+    hit_mask = ids[:, 18] != 0xFFFFFFFF
+    # a miss leaves tfar at its input, +inf: the files carry hit / miss in `hit` and 0 as the tfar of a miss, so that every value is finite
+    fields = {"ray_index": idx.astype(np.float64), "ray_org": ray[:, 0:3], "ray_tnear": ray[:, 3], "ray_dir": ray[:, 4:7],
+              "hit": hit_mask.astype(np.float32), "tfar": np.where(hit_mask, hit[:, 8], np.float32(0)),
+              "Ng": hit[:, 12:15], "u": hit[:, 15], "v": hit[:, 16],
+              "primID": ids[:, 17].astype(np.float64), "geomID": ids[:, 18].astype(np.float64), "instID": ids[:, 19].astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in fields.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+    log(f"wrote {len(fields)} arrays of {k} sampled rays to {out_dir}")
 
 
 def emit(line):

@@ -3,7 +3,7 @@ ROOT='/root/repo'
 for t in (0,1,2):
     out=f'/tmp/hair_{t}.raw'
     t0=time.time()
-    r=subprocess.run([os.path.join(ROOT,'tests/link_compat/_bin/embree_hair_geometry'),out,'96','72','4',str(t),'3000'],stdout=subprocess.PIPE,stderr=subprocess.STDOUT,text=True,timeout=600)
+    r=subprocess.run([os.path.join(ROOT,'oracle/_ref/link_compat/embree_hair_geometry'),out,'96','72','4',str(t),'3000'],stdout=subprocess.PIPE,stderr=subprocess.STDOUT,text=True,timeout=600)
     dt=time.time()-t0
     print(r.returncode, r.stdout.strip()[-300:], "%.1fs"%dt)
     g=np.fromfile(out,np.uint32); w=np.fromfile(os.path.join(ROOT,f'tests/golden/hair_geometry_{t}_96x72.raw'),np.uint32)

@@ -364,7 +364,29 @@ def main():
     main_filters()
 
 
+def main_abi():
+    """reference_abi.json: tests/test_abi.py's layout probe compiled against the reference headers (with the rtcore_config.h that
+    oracle/build_ref.py generates) and the prototypes of every rtc* function they declare; the reference is where
+    oracle/build_ref.py finds it."""
+    import glob
+    import json
+    from tests import test_abi
+    sys.path.insert(0, os.path.join(ROOT, "oracle"))
+    from build_ref import REF as ref_dir
+    probe = test_abi._probe("embree4/rtcore.h", extra_inc=(os.path.join(ref_dir, "include"),
+                                                          os.path.join(ROOT, "oracle", "_ref", "gen_rel", "include", "embree4")))
+    protos = {}
+    for f in sorted(glob.glob(os.path.join(ref_dir, "include", "embree4", "*.h"))):
+        protos.update(test_abi._prototypes(open(f).read()))
+    rows = [f"  {json.dumps(k)}: {json.dumps(list(v))}" for k, v in sorted(protos.items())]
+    with open(os.path.join(HERE, "reference_abi.json"), "w") as f:
+        f.write('{"layout_probe": ' + json.dumps(probe) + ',\n "prototypes": {\n' + ",\n".join(rows) + "\n }}\n")
+
+
 if __name__ == "__main__":
+    if len(sys.argv) > 1 and sys.argv[1] == "abi":
+        main_abi()
+        sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "curves":
         main_curves()
         sys.exit(0)

@@ -144,6 +144,49 @@ def load_reference():
     return _ref
 
 
+REFERENCE_RUNS = os.path.join(ROOT, "tests", "golden", "reference_runs")
+HIT_FIELDS = ("tfar", "Ng_x", "Ng_y", "Ng_z", "u", "v", "primID", "instID", "instPrimID")
+
+
+def sample_rays(rays, n=576):
+    """A seeded random sample of n rays, in stream order: the rays a reference-run fixture holds outputs for.  (A stride
+    would alias with the tests' periodic patterns -- ray masks by index mod 4, tfar on every 7th ray.)"""
+    idx = np.sort(np.random.default_rng(0).choice(len(rays), min(n, len(rays)), replace=False))
+    return rays[idx].copy()
+
+
+def reference_run(case, rays, run):
+    """The unmodified reference's (rtcIntersect1 records, rtcOccluded1 records, extras) for `rays`, read from
+    tests/golden/reference_runs/<case>.npz.  With RTCB200_RECORD_REFERENCE=1 and oracle/_ref built, run(R) computes them
+    with the reference library R first and rewrites the fixture (extras: a dict of small arrays, e.g. scene bounds).
+    The file keeps geomID for every ray, the other hit fields for the rays that hit, and one occluded bit per ray: a miss
+    leaves the RTCRayHit record as it came in, a ray that is not occluded keeps its tfar (checked when recording)."""
+    import hashlib
+    from embree_b200.rtc import rays_of
+    path = os.path.join(REFERENCE_RUNS, case + ".npz")
+    digest = np.frombuffer(hashlib.sha256(rays.tobytes()).digest(), np.uint8)
+    if os.environ.get("RTCB200_RECORD_REFERENCE"):
+        R = load_reference()
+        assert R is not None, "RTCB200_RECORD_REFERENCE needs oracle/_ref (python oracle/build_ref.py)"
+        hit, occ, extras = run(R)
+        h = hit["geomID"] != 0xFFFFFFFF
+        o = occ["tfar"] == -np.inf
+        assert hit[~h].tobytes() == rays[~h].tobytes(), f"{case}: the reference changed the record of a miss"
+        assert occ[~o].tobytes() == rays_of(rays)[~o].tobytes(), f"{case}: the reference changed a ray that is not occluded"
+        os.makedirs(REFERENCE_RUNS, exist_ok=True)
+        np.savez_compressed(path, rays_sha256=digest, geomID=hit["geomID"], occluded=np.packbits(o),
+                            **{f: hit[f][h] for f in HIT_FIELDS}, **{"x_" + k: np.asarray(v) for k, v in extras.items()})
+    z = np.load(path)
+    assert (z["rays_sha256"] == digest).all(), f"{case}: the test's rays no longer reproduce the rays of the fixture"
+    hit, occ = rays.copy(), rays_of(rays)
+    hit["geomID"] = z["geomID"]
+    h = hit["geomID"] != 0xFFFFFFFF
+    for f in HIT_FIELDS:
+        hit[f][h] = z[f]
+    occ["tfar"][np.unpackbits(z["occluded"], count=len(rays)).astype(bool)] = -np.inf
+    return hit, occ, {k[2:]: z[k] for k in z.files if k.startswith("x_")}
+
+
 def api_trace_mt(lib, scene, recs, nthreads, K=1, occluded=False, coherent=False, valid=None):
     """Loop lib's rtcIntersect1 / rtcOccluded1 / rtcIntersect{K} over `recs` on `nthreads` host threads (FTZ|DAZ set),
     i.e. how a host application drives the reference (BASELINE.md section 4)."""

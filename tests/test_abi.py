@@ -1,6 +1,6 @@
 """Drop-in boundary checks that need no GPU: the product library loads, exports every symbol that
-include/embree4_b200.h declares, the POD layouts equal the reference's (measured values from SURVEY 8b and, when
-the reference headers are available in this container, compiled side by side), and the library fails loudly --
+include/embree4_b200.h declares, the POD layouts equal the reference's (measured values from SURVEY 8b and the
+same probe compiled against the reference headers, tests/golden/reference_abi.json), and the library fails loudly --
 it has no CPU fallback -- when no CUDA device exists."""
 import ctypes as C
 import os
@@ -57,11 +57,13 @@ def test_layout_matches_reference_values():
     # sizeof(RTCRay)=48, RTCHit=48, RTCRayHit=96, offsetof(hit)=48, RTCRayHit4/8/16 = 336/672/1344 (SURVEY 8b, measured)
     assert got[:7] == ["48", "48", "96", "48", "336", "672", "1344"]
     assert got[7] == "768" and got[8] == "768"
-    ref_inc = "/root/reference/include"
-    gen = os.path.join(ROOT, "oracle", "_ref", "gen_rel", "include", "embree4")
-    if os.path.exists(os.path.join(ref_inc, "embree4", "rtcore.h")) and os.path.exists(gen):
-        want = _probe("embree4/rtcore.h", extra_inc=(ref_inc, gen))
-        assert got == want
+    assert got == _reference_abi()["layout_probe"]   # the same probe compiled against the reference's headers
+
+
+def _reference_abi():
+    """tests/golden/reference_abi.json (make_golden.py abi): the probe's output and every rtc* prototype of the reference headers."""
+    import json
+    return json.load(open(os.path.join(ROOT, "tests", "golden", "reference_abi.json")))
 
 
 def _declared_symbols():
@@ -164,13 +166,7 @@ def _prototypes(text):
 def test_prototypes_match_the_reference_headers():
     """Every rtc* function include/embree4_b200.h declares has the reference's signature (return type, parameter types and order,
     include/embree4/rtcore_*.h); the reference functions the header does not declare are exactly the stubs outside the path."""
-    import glob
-    ref_dir = "/root/reference/include/embree4"
-    if not os.path.isdir(ref_dir):
-        pytest.skip("reference headers not present")
-    ref = {}
-    for f in glob.glob(os.path.join(ref_dir, "*.h")):
-        ref.update(_prototypes(open(f).read()))
+    ref = {n: (r, p) for n, (r, p) in _reference_abi()["prototypes"].items()}
     mine = _prototypes(open(HEADER).read())
     shared = [n for n in mine if n in ref]
     assert len(shared) >= 85

@@ -1,17 +1,19 @@
 """The reference's own tutorial (tutorials/minimal/minimal.cpp), compiled unmodified against the reference's own
-headers, linked against libembree4_b200.so (tests/link_compat/build.sh): existing callers link unchanged."""
+headers, linked against libembree4_b200.so (oracle/build_link_compat.sh, which build() runs where the reference is present;
+the binaries live in oracle/_ref/link_compat with the other reference build products): existing callers link unchanged."""
 import os
 import subprocess
 
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EXE = os.path.join(ROOT, "tests", "link_compat", "_bin", "embree_minimal")
+BIN = os.path.join(ROOT, "oracle", "_ref", "link_compat")
+EXE = os.path.join(BIN, "embree_minimal")
 LIB = os.path.join(ROOT, "embree_b200", "csrc", "libembree4_b200.so")
 
 
 def _ensure_built():
-    subprocess.check_call([os.path.join(ROOT, "tests", "link_compat", "build.sh")])
+    subprocess.check_call([os.path.join(ROOT, "oracle", "build_link_compat.sh")])
     if not os.path.exists(EXE):
         pytest.skip("reference sources not available and no prebuilt binary")
 
@@ -37,7 +39,7 @@ def test_reference_tutorial_runs_on_the_gpu():
     assert "Did not find any intersection." in out, out
 
 
-TUT = os.path.join(ROOT, "tests", "link_compat", "_bin", "embree_triangle_geometry")
+TUT = os.path.join(BIN, "embree_triangle_geometry")
 GOLDEN_FRAME = os.path.join(ROOT, "tests", "golden", "triangle_geometry_160x120.raw")
 
 
@@ -68,7 +70,7 @@ def test_triangle_geometry_tutorial_renders_the_reference_frame(tmp_path):
     assert diff.sum() <= 0.003 * w.size and not (diff & ~edge).any(), f"{diff.sum()} pixels differ, {(diff & ~edge).sum()} of them off an edge"
 
 
-POINTS = os.path.join(ROOT, "tests", "link_compat", "_bin", "embree_point_geometry")
+POINTS = os.path.join(BIN, "embree_point_geometry")
 
 
 @pytest.mark.gpu
@@ -99,7 +101,7 @@ def test_point_geometry_tutorial_renders_the_reference_frame(tmp_path):
     assert big.sum() <= 0.005 * w.size and diff.sum() <= 0.03 * w.size and not (big & ~edge).any(), f"{diff.sum()} pixels differ, {big.sum()} by more than one step, {(big & ~edge).sum()} of them off an edge"
 
 
-HAIR = os.path.join(ROOT, "tests", "link_compat", "_bin", "embree_hair_geometry")
+HAIR = os.path.join(BIN, "embree_hair_geometry")
 
 
 @pytest.mark.gpu
@@ -137,7 +139,7 @@ def test_hair_geometry_tutorial_renders_the_reference_frame(tmp_path, ctype, nam
         assert same >= 0.93 and mean_diff < 1.0, (name, same, mean_diff)
 
 
-DYN = os.path.join(ROOT, "tests", "link_compat", "_bin", "embree_dynamic_scene")
+DYN = os.path.join(BIN, "embree_dynamic_scene")
 
 
 @pytest.mark.gpu
